@@ -2,6 +2,7 @@
 """bench.py — BASELINE.json metric on the BASELINE configs, one JSON line on stdout (rank 0).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--only infer,train,spp_nms,nms,lib,cpu]
+                  [--dump-outputs DIR]
   torchrun ... bench.py --gpus N ...        (one rank per GPU)
 
 Headline (config 2, `metric`/`value`/`e2e`/`roofline`): a step = one pass of the hot path (Model.forward + Detect decode,
@@ -19,7 +20,9 @@ Extra keys (the other BASELINE configs, tools/bench_workloads.py):
   nms        config 5: five thresholds x single/multi-label on synthetic [32,25200,85]
   gpu_library_baseline   the reference itself on this GPU through PyTorch+cuDNN / torchvision / torch DDP (informational)
   cpu_baseline / --impl reference: the reference's own torch-CPU Model + non_max_suppression from the staged copy
-             (baseline/_ref, kind "reference"), else the oracle port (kind "port"), on the host cores, bounded sample.
+             (oracle/_ref, kind "reference"), else the oracle port (kind "port"), on the host cores, bounded sample.
+The timed loop of every leg runs --steps steps.  --dump-outputs DIR writes what the headline's timed forward returned in its last step
+(dump_outputs); the inputs and weights are seeded, so two builds run with the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -44,6 +47,7 @@ GFLOP_LAYER0 = 0.708             # layer 0 runs on CUDA cores (c_in=3); excluded
 METRIC = "images/sec @640 bs32 YOLOv3"
 UNIT = "images/s"
 PARITY_TOL = 2e-2
+DUMP_ROWS = 65536  # rows of z and of the head logits that --dump-outputs writes: 2 x 22 MB
 
 
 def peaks():
@@ -129,6 +133,27 @@ class ClockSampler:
                     reasons=sorted(reasons), samples=len(sm))
 
 
+def sample_outputs(z, raw):
+    """A fixed, seeded sample of what the timed forward returns: rows of z [bs, rows, 85] (decoded boxes) and the same rows
+    of the Detect head's logits p_i [bs, na, ny, nx, 85] (row r of image b in z is decoded from logits row r of image b,
+    rows ordered level, anchor, y, x).  ``sample_rows`` holds the flat indices b * rows + r, as float64."""
+    import torch
+
+    n, rows, no = z.shape
+    idx = torch.randperm(n * rows, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    logits = torch.cat([p.reshape(n, -1, no) for p in raw], 1).reshape(n * rows, no)
+    di = idx.to(z.device)
+    return {"z": z.reshape(n * rows, no)[di].cpu().numpy(), "raw": logits[di].cpu().numpy(), "sample_rows": idx.double().numpy()}
+
+
+def dump_outputs(out_dir: Path, arrays):
+    import numpy as np
+
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def aggregate(ms_local: float, dev) -> float:
     """Max over ranks of a locally event-timed duration (one process per GPU; NCCL on GPUs, gloo in the CPU tests)."""
     import torch
@@ -163,7 +188,7 @@ def build_model(device):
 # ------------------------------------------------------------------------------------------ CPU legs (checker / baseline only)
 class CpuReference:
     """The reference's torch-CPU forward for the bench model: the reference's OWN ``Model`` from the staged copy
-    (baseline/_ref, ``kind = "reference"``) when present, else the oracle port (``kind = "port"``), holding the same weights
+    (oracle/_ref, ``kind = "reference"``) when present, else the oracle port (``kind = "port"``), holding the same weights
     as the GPU model (``params``), fused, fp32, inference mode.  Thread count: calibrated AT the batch that is timed."""
 
     def __init__(self, params=None):
@@ -296,7 +321,7 @@ def library_baseline(dev, rank, world, bs=32, img=640, steps=10, train_bs=8):
     torch.optim.SGD under bf16 autocast.  Informational: this is the bar a kernel library sets on the same hardware."""
     shim = _reference_modules()
     if shim is None:
-        return {"unavailable": "reference not staged (baseline/_ref missing: run oracle/stage_reference.py in the build container)"}
+        return {"unavailable": "reference not staged (oracle/_ref missing: see oracle/stage_reference.py)"}
     from models.yolo import Model as RefModel
     from utils.general import non_max_suppression as ref_nms
     from utils.loss import ComputeLoss as RefLoss
@@ -379,12 +404,11 @@ def library_baseline(dev, rank, world, bs=32, img=640, steps=10, train_bs=8):
         if world > 1:
             dist.barrier()
         e0.record()
-        n = max(3, steps // 2)
-        for _ in range(n):
+        for _ in range(steps):
             step()
         e1.record()
         torch.cuda.synchronize()
-        ms = aggregate(e0.elapsed_time(e1) / n, dev)
+        ms = aggregate(e0.elapsed_time(e1) / steps, dev)
         res["train"] = {"images_per_s": world * train_bs / (ms / 1e3), "ms_per_step": ms, "batch_per_gpu": train_bs,
                         "what": "reference Model + ComputeLoss, torch.autocast(bf16), DistributedDataParallel (NCCL), clip + torch SGD; "
                                 "no EMA, no H2D"}
@@ -403,6 +427,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only", default="all", help="comma list of legs besides the headline: train,spp_nms,nms,lib,cpu (default all)")
     ap.add_argument("--per-op", default=None, help="write the per-launch timing table (JSON) to this path")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write a seeded sample of the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     legs = {"train", "spp_nms", "nms", "lib", "cpu"} if args.only == "all" else set(filter(None, args.only.split(","))) - {"none"}
@@ -462,6 +488,7 @@ def main():
     e1.record()
     torch.cuda.synchronize()
     ms_total = e0.elapsed_time(e1)
+    dumped = sample_outputs(eng.z, eng.raw) if args.dump_outputs and rank == 0 else None
     clocks = None
     if rank == 0:
         # the clock samples must come from this workload: keep replaying it (untimed) until >= 0.6 s of load were observed
@@ -519,7 +546,7 @@ def main():
     if rank == 0:
         from yolov3_b200.profile import time_ops
 
-        per_op = time_ops(eng, xs[0], iters=max(3, min(10, args.steps)))
+        per_op = time_ops(eng, xs[0], iters=args.steps)
     del pipe, graphs
     model._engines.clear()
     del eng
@@ -543,13 +570,13 @@ def main():
     if "nms" in legs:
         leg("nms", lambda: {"workload": f"synthetic [bs {BS}/GPU, 25200, 85] fp32 (SURVEY §8d config 5), max_det 300, device-resident, "
                                         "sync-free y3_nms_batched; iou 0.6 at conf <= 0.01 else 0.45", "unit": "input boxes/s",
-                            **W.nms_sweep_workload(dev, rank, world, bs=BS)})
+                            **W.nms_sweep_workload(dev, rank, world, bs=BS, reps=args.steps)})
     if "spp_nms" in legs:
-        leg("spp_nms", lambda: W.spp_nms_workload(dev, rank, world, bs=8, img=IMG, steps=max(10, args.steps), warmup=args.warmup))
+        leg("spp_nms", lambda: W.spp_nms_workload(dev, rank, world, bs=8, img=IMG, steps=args.steps, warmup=args.warmup))
     if "train" in legs:
-        leg("train", lambda: W.train_step_workload(dev, rank, world, bs=8, img=IMG, steps=max(5, min(10, args.steps)), warmup=3))
+        leg("train", lambda: W.train_step_workload(dev, rank, world, bs=8, img=IMG, steps=args.steps, warmup=3))
     if "lib" in legs:
-        leg("gpu_library_baseline", lambda: library_baseline(dev, rank, world, bs=BS, img=IMG, steps=max(5, min(10, args.steps))))
+        leg("gpu_library_baseline", lambda: library_baseline(dev, rank, world, bs=BS, img=IMG, steps=args.steps))
 
     if rank != 0:
         if world > 1:
@@ -589,7 +616,7 @@ def main():
         cpu = {"value": probe.shape[0] / dt, "unit": UNIT, "cores": ref.threads, "kind": ref.kind,
                "sample": f"8 of the {BS} images of a step, one timed pass after warm-up and thread calibration "
                          f"(img/s by thread count: {ref.tried}); "
-                         + ("reference models.yolo.Model from baseline/_ref" if ref.kind == "reference" else "oracle port")}
+                         + ("reference models.yolo.Model from oracle/_ref" if ref.kind == "reference" else "oracle port")}
         zr = z_ref[:n_par].double()
         parity = float((z_par.double() - zr).norm() / zr.norm())
 
@@ -609,6 +636,8 @@ def main():
         "clocks": clocks,
         **extra,
     }
+    if dumped is not None:
+        dump_outputs(Path(args.dump_outputs), dumped)
     print(json.dumps(line), flush=True)
     if not z_finite or (parity is not None and not parity <= PARITY_TOL):
         print(f"bench: PARITY FAILURE: rel-L2 {parity} (tolerance {PARITY_TOL}), finite {z_finite}", file=sys.stderr)

@@ -10,10 +10,10 @@ here from the published ultralytics 8.x formulas (SURVEY.md Appendix B) and unit
 ``tests/golden/make_golden.py`` (``gen_iou``: float64 CIoU cross-check, ``torchvision.ops.box_iou``; ``gen_forward``: fused
 vs unfused forward through ``fuse_conv_and_bn``) and re-checked from the fixtures by ``tests/test_oracle_golden.py``.
 
-Consumers: ``tests/golden/make_golden.py`` (golden-vector generation in the build container, reference at
-``/root/reference``); ``bench.py --impl reference`` / its ``cpu_baseline`` leg and ``tests/test_zz_reference_seam_gpu.py``,
-which run the reference from the byte-for-byte staged copy ``baseline/_ref/`` (``oracle/stage_reference.py``; git-ignored,
-travels to the GPU box with the snapshot).  Nothing under ``yolov3_b200/`` imports this.
+Consumers: ``tests/golden/make_golden.py`` (golden-vector generation, pointed at a checkout of the reference with
+``--reference``) and ``bench.py``'s reference legs, which run the byte-for-byte copy that ``build()`` stages under the
+git-ignored ``oracle/_ref/`` (``oracle/stage_reference.py``) when a reference checkout is at hand.  No test reads the
+reference: what they compare against is stored under ``tests/golden/``.  Nothing under ``yolov3_b200/`` imports this.
 """
 from __future__ import annotations
 
@@ -30,8 +30,8 @@ import torch
 import torch.nn as nn
 
 _REPO = Path(__file__).resolve().parents[1]
-# the read-only checkout in the build container, else the staged copy that ships to the GPU box
-REFERENCE_ROOT = Path("/root/reference") if (Path("/root/reference") / "models" / "yolo.py").exists() else _REPO / "baseline" / "_ref"
+# the copy build() stages (oracle/stage_reference.py); make_golden.py points this at a reference checkout instead
+REFERENCE_ROOT = _REPO / "oracle" / "_ref"
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -412,7 +412,7 @@ def _module(name, **attrs):
 
 
 def install():
-    """Register the stand-in modules and put ``/root/reference`` on sys.path.  Idempotent."""
+    """Register the stand-in modules and put ``REFERENCE_ROOT`` on sys.path.  Idempotent."""
     if "ultralytics" in sys.modules and getattr(sys.modules["ultralytics"], "_y3_shim", False):
         return
     noop = lambda *a, **k: None  # noqa: E731

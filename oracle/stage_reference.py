@@ -1,17 +1,16 @@
-"""TEST / BASELINE INFRASTRUCTURE ONLY — stages the UNMODIFIED reference (ultralytics/yolov3, read-only at /root/reference)
-under the git-ignored ``baseline/_ref/`` so that it travels to the GPU box with the repo snapshot (``/root/reference`` does
-not exist there).  Nothing under ``yolov3_b200/`` ever imports it; the only consumers are ``bench.py --impl reference`` /
-``bench.py``'s ``cpu_baseline`` leg (the reference's own ``Model`` / ``non_max_suppression`` timed on the host cores) and the
-seam test ``tests/test_zz_reference_seam_gpu.py`` (the reference's detect/val loop bodies with our backend swapped in).
+"""BASELINE INFRASTRUCTURE ONLY — stages the UNMODIFIED reference (ultralytics/yolov3 @ 97b87b1) under the git-ignored
+``oracle/_ref/`` when a checkout of it is at hand, so that a built tree carries it to machines that have none.  Nothing
+under ``yolov3_b200/`` and no test imports it; the only consumers are ``bench.py --impl reference`` / ``bench.py``'s
+``cpu_baseline`` leg (the reference's own ``Model`` / ``non_max_suppression`` timed on the host cores) and its
+``gpu_library_baseline`` leg.  Without it they fall back to the oracle port or report themselves unavailable.
 
-Why a file copy and not ``pip install --target baseline/_ref /root/reference``: tried (round 2) — the reference's
-pyproject.toml declares no ``version`` (setuptools: "`project` must contain ['version'] properties") and its layout is a
-flat script tree (``models/``, ``utils/``, ``detect.py`` at top level: not an installable distribution), so metadata
-generation fails before anything is built.  The reference is meant to be run from a clone (its README); a clone of the
-needed files is what this makes.  Files are copied byte for byte, never edited; ``baseline/_ref/`` is listed in .gitignore so
-no reference source enters this repository's history.
+Why a file copy and not ``pip install --target``: the reference's pyproject.toml declares no ``version`` (setuptools:
+"`project` must contain ['version'] properties") and its layout is a flat script tree (``models/``, ``utils/``,
+``detect.py`` at top level: not an installable distribution), so metadata generation fails before anything is built.  The
+reference is meant to be run from a clone (its README); a clone of the needed files is what this makes.  Files are copied
+byte for byte, never edited; ``oracle/_ref/`` is listed in .gitignore so no reference source enters this repository.
 
-    python oracle/stage_reference.py            # no-op when /root/reference is absent (GPU box) or already staged
+    python oracle/stage_reference.py            # no-op when no reference checkout is present or it is already staged
 """
 from __future__ import annotations
 
@@ -21,7 +20,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parents[1]
 SRC = Path("/root/reference")
-DST = ROOT / "baseline" / "_ref"
+DST = ROOT / "oracle" / "_ref"
 # what the hot path's callers import: the model/graph code, the utils they pull in, the three loop scripts, YAMLs, the two
 # sample images of BASELINE config 1 and the hyper-parameter files ComputeLoss reads
 TOP_FILES = ["detect.py", "val.py", "train.py", "hubconf.py", "export.py", "LICENSE"]
@@ -33,8 +32,15 @@ def staged() -> bool:
     return (DST / "models" / "yolo.py").exists()
 
 
+def source_available() -> bool:
+    try:
+        return (SRC / "models" / "yolo.py").exists()
+    except OSError:  # a checkout the building user may not read: nothing to stage
+        return False
+
+
 def stage(force: bool = False) -> Path | None:
-    if not (SRC / "models" / "yolo.py").exists():
+    if not source_available():
         return DST if staged() else None
     if staged() and not force:
         return DST

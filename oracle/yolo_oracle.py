@@ -177,6 +177,18 @@ def init_params(cfg, seed=0, randomize_bn=True, ch=3):
     return p
 
 
+def confident_params(cfg, seed=0):
+    """``init_params`` with the objectness / class biases raised so that detections exist at ordinary thresholds (the
+    shipped init gives conf ~ 3e-5 everywhere: nothing to compare)."""
+    p = init_params(cfg, seed=seed)
+    for k in p:
+        if ".m." in k and k.endswith(".bias"):
+            b = p[k].view(3, -1)
+            b[:, 4] += 7.0   # sigmoid(-3.9 .. -5.3 + 7) = 0.85 .. 0.96
+            b[:, 5:] += 5.0  # sigmoid(-4.9 + 5 +- noise) ~ 0.5: obj * cls crosses 0.25 for a share of the classes
+    return p
+
+
 def fold_bn(w, gamma, beta, mean, var, eps=BN_EPS):
     """fuse_conv_and_bn (ultralytics; semantic of models/yolo.py:163-172): W'=diag(g/sqrt(var+eps))W, b'=beta-g*mean/sqrt(var+eps)."""
     scale = gamma / torch.sqrt(var + eps)

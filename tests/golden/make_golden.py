@@ -1,8 +1,10 @@
-"""Generate the golden fixtures in tests/golden/ by running the REFERENCE ITSELF (/root/reference, imported unmodified
-through oracle/ref_shim.py) on seeded inputs, and assert that the CPU oracle (oracle/yolo_oracle.py) agrees with it.
+"""Generate the golden fixtures in tests/golden/ by running the REFERENCE ITSELF (a checkout of ultralytics/yolov3 @ 97b87b1,
+imported unmodified through oracle/ref_shim.py) on seeded inputs, and assert that the CPU oracle (oracle/yolo_oracle.py)
+agrees with it.
 
-Run in the build container only (the GPU box has no /root/reference):   python tests/golden/make_golden.py
-The fixtures it writes are committed; tests/test_oracle_golden.py re-checks the oracle against them everywhere.
+    python tests/golden/make_golden.py --reference <checkout> [iou nms loss forward scale val tta seam]
+
+The fixtures it writes are committed; the tests compare against them and never read the reference.
 
 What is pinned (SURVEY.md Appendix D):
   forward_<model>.npz   Model.forward (fused and unfused) -> z, raw p_i, layer taps      (models/yolo.py:135-147, 89-123)
@@ -11,6 +13,7 @@ What is pinned (SURVEY.md Appendix D):
   iou_cases.npz         box_iou, bbox_iou(CIoU) values                                    (ultralytics, via shim)
   val_cases.npz         val.process_batch correct[N,10] on seeded detections / labels     (val.py:147-188)
   tta_cases.npz         Model.forward(x, augment=True) rows (scale / flip views merged)    (models/yolo.py:239-280)
+  seam_cases.npz        detect.py / val.py loop pieces, smart_optimizer groups, letterbox (see gen_seam)
 """
 from __future__ import annotations
 
@@ -319,11 +322,111 @@ def gen_val():
     np.savez_compressed(OUT / "val_cases.npz", **store)
 
 
+SEAM_IMGSZ = 128  # detect.py's image size for the seam fixture: small enough to store its inputs and predictions
+LETTERBOX_SHAPES = [(1080, 810), (375, 500), (333, 1000)]
+LETTERBOX_KW = [dict(auto=True), dict(auto=False), dict(auto=False, scaleFill=True), dict(auto=True, scaleup=False)]
+
+
+def gen_seam():
+    """What the seam tests (tests/test_zz_reference_seam_gpu.py, tests/test_params_cpu.py, tests/test_oracle_golden.py)
+    compare against:
+      detect/<i>/*     detect.py:166-223 on data/images with yolov3-tiny (confident weights): LoadImages' letterboxed input,
+                       Model forward z, non_max_suppression(0.25, 0.45, max_det=50), scale_boxes to the native image
+      val/<si>/*       val.py:355-390 on synthetic predictions: NMS(0.001, 0.6, multi-label), scale_boxes, process_batch
+      optim/<cfg>/<g>  smart_optimizer(SGD, 0.01, 0.937, 5e-4) (utils/torch_utils.py:207-237): parameter names per group and
+                       (lr, momentum, dampening, weight_decay, nesterov)
+      letterbox/<i>_<k>  utils/augmentations.py letterbox on seeded random images: sha256 of the image, ratio, pad"""
+    import hashlib
+
+    import utils.general as G  # reference
+    import val as V  # reference
+    from models.yolo import Model  # reference
+    from utils.augmentations import letterbox  # reference
+    from utils.dataloaders import LoadImages  # reference
+    from utils.torch_utils import smart_optimizer  # reference
+
+    sys.path.insert(0, str(ROOT))
+    from yolov3_b200.module import DetectionModel
+
+    store = {}
+    real_time = G.time.time
+    G.time.time = lambda: 0.0  # disable the wall-clock time_limit break (utils/general.py:675,746-748)
+    try:
+        params = O.confident_params(CFG / "yolov3-tiny.yaml")
+        m = ref_model("yolov3-tiny", params)
+        images = LoadImages(str(ref_shim.REFERENCE_ROOT / "data" / "images"), img_size=(SEAM_IMGSZ, SEAM_IMGSZ), stride=32, auto=True)
+        for i, (path, im, im0s, _, _) in enumerate(images):
+            x = torch.from_numpy(im).float()[None] / 255
+            with torch.no_grad():
+                z = m(x)[0]
+            det = G.non_max_suppression(z.clone(), 0.25, 0.45, max_det=50)[0]
+            assert len(det) >= 1, path
+            # bit-equal confidences are ordered by an unstable argsort in the reference and by index in the oracle (and in
+            # yolov3_b200): the fixture must not depend on that order, i.e. both keep the same set of rows
+            (ora,), _ = O.non_max_suppression(z.clone(), 0.25, 0.45, max_det=50)
+            a = det.numpy()
+            assert np.array_equal(a[np.lexsort(a.T[::-1])], ora[np.lexsort(ora.T[::-1])]), path
+            store[f"detect/{i}/im"], store[f"detect/{i}/im0_shape"] = im, np.array(im0s.shape)
+            store[f"detect/{i}/z"], store[f"detect/{i}/det"] = z.numpy(), a
+            store[f"detect/{i}/scaled"] = G.scale_boxes(x.shape[2:], det[:, :4].clone(), im0s.shape).numpy()
+            print("seam detect", Path(path).name, tuple(im.shape), len(det))
+
+        pred = O.synth_predictions(2, n_rows=3000, nc=80, seed=5)
+        targets = O.synth_targets(2, seed=4)
+        h = w = 640
+        shape0, ratio_pad = (480, 600), ((1.0667, 1.0667), (0.0, 64.0))
+        targets[:, 2:] *= torch.tensor((w, h, w, h))
+        iouv = torch.linspace(0.5, 0.95, 10)
+        out = G.non_max_suppression(pred.clone(), 0.001, 0.6, multi_label=True, max_det=300)
+        for si in range(2):
+            labels = targets[targets[:, 0] == si, 1:]
+            predn = out[si].clone()
+            G.scale_boxes((h, w), predn[:, :4], shape0, ratio_pad)
+            tbox = G.xywh2xyxy(labels[:, 1:5])
+            G.scale_boxes((h, w), tbox, shape0, ratio_pad)
+            labelsn = torch.cat((labels[:, 0:1], tbox), 1)
+            store[f"val/{si}/out"], store[f"val/{si}/predn"] = out[si].numpy(), predn.numpy()
+            store[f"val/{si}/labelsn"], store[f"val/{si}/correct"] = labelsn.numpy(), V.process_batch(predn, labelsn, iouv).numpy()
+    finally:
+        G.time.time = real_time
+
+    for name in ("yolov3", "yolov3-tiny"):
+        groups = []
+        for model in (Model(str(ref_shim.REFERENCE_ROOT / "models" / f"{name}.yaml")), DetectionModel(CFG / f"{name}.yaml", device="cpu")):
+            by_ptr = {p.data_ptr(): n for n, p in model.named_parameters()}
+            opt = smart_optimizer(model, "SGD", 0.01, 0.937, 5e-4)
+            groups.append([(sorted(by_ptr[p.data_ptr()] for p in g["params"]),
+                            [g["lr"], g["momentum"], g["dampening"], g["weight_decay"], float(g["nesterov"])]) for g in opt.param_groups])
+        assert groups[0] == groups[1], name  # the reference's own Model and the nn.Module facade group alike
+        for gi, (names, hyp) in enumerate(groups[0]):
+            store[f"optim/{name}/{gi}/names"], store[f"optim/{name}/{gi}/hyp"] = np.array(names), np.array(hyp)
+        print("seam optim", name, [len(n) for n, _ in groups[0]])
+
+    rng = np.random.default_rng(1)
+    store["letterbox/shapes"], store["letterbox/kw"] = np.array(LETTERBOX_SHAPES), np.array(repr(LETTERBOX_KW))
+    for i, (h, w) in enumerate(LETTERBOX_SHAPES):
+        im = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
+        for k, kw in enumerate(LETTERBOX_KW):
+            a = letterbox(im.copy(), **kw)
+            store[f"letterbox/{i}_{k}/sha256"] = np.array(hashlib.sha256(np.ascontiguousarray(a[0]).tobytes()).hexdigest())
+            store[f"letterbox/{i}_{k}/shape"] = np.array(a[0].shape)
+            store[f"letterbox/{i}_{k}/ratio"], store[f"letterbox/{i}_{k}/pad"] = np.array(a[1], np.float64), np.array(a[2], np.float64)
+    np.savez_compressed(OUT / "seam_cases.npz", **store)
+    print("seam ok")
+
+
 if __name__ == "__main__":
-    assert ref_shim.reference_available(), "run in the build container: /root/reference is required"
+    args = sys.argv[1:]
+    if "--reference" in args:
+        i = args.index("--reference")
+        ref_shim.REFERENCE_ROOT = Path(args[i + 1]).resolve()
+        del args[i:i + 2]
+    assert ref_shim.reference_available(), "pass --reference <checkout of ultralytics/yolov3 @ 97b87b1>"
     ref_shim.install()
     torch.set_num_threads(8)
-    which = sys.argv[1:] or ["iou", "nms", "loss", "forward", "scale", "val", "tta"]
+    which = args or ["iou", "nms", "loss", "forward", "scale", "val", "tta", "seam"]
+    if "seam" in which:
+        gen_seam()
     if "tta" in which:
         gen_tta()
     if "val" in which:

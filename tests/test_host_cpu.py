@@ -309,7 +309,7 @@ def test_reference_arm_json_contract():
     assert d["higher_is_better"] is True and d["steps"] == 1 and d["value"] > 0 and d["n_gpus"] == 2
     assert d["config"]["global_batch"] == 64
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
-    # the reference's own Model from the staged copy (baseline/_ref) when it is there, else the oracle port — and it says which
+    # the reference's own Model from the staged copy (oracle/_ref) when it is there, else the oracle port — and it says which
     sys.path.insert(0, str(root / "oracle"))
     import ref_shim
 

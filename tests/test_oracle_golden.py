@@ -148,8 +148,9 @@ def test_process_batch_oracle_vs_reference_golden():
 
 def test_letterbox_oracle_vs_cv2_and_reference():
     """oracle.resize_linear_u8 / letterbox (restating OpenCV's 8-bit INTER_LINEAR and utils/augmentations.py:104-134) against
-    cv2 itself (third-party, installed: opencv-python 4.13) and, when the reference is importable, its own letterbox()."""
-    import sys
+    cv2 itself (third-party, installed: opencv-python 4.13) and the reference's own letterbox() (seam_cases.npz: digest of
+    its image, ratio and padding on seeded random images)."""
+    import hashlib
 
     cv2 = pytest.importorskip("cv2")
     rng = np.random.default_rng(0)
@@ -157,15 +158,12 @@ def test_letterbox_oracle_vs_cv2_and_reference():
                            (501, 333, 417, 277), (64, 64, 200, 31), (33, 77, 32, 75)]:
         im = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
         assert np.array_equal(O.resize_linear_u8(im, nw, nh), cv2.resize(im, (nw, nh), interpolation=cv2.INTER_LINEAR)), (h, w, nh, nw)
-    sys.path.insert(0, str(Path(__file__).resolve().parents[1] / "oracle"))
-    import ref_shim
-
-    if ref_shim.reference_available():
-        ref_shim.install()
-        from utils.augmentations import letterbox as ref_letterbox
-
-        for (h, w) in [(1080, 810), (375, 500), (333, 1000)]:
-            im = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-            for kw in [dict(auto=True), dict(auto=False), dict(auto=False, scaleFill=True), dict(auto=True, scaleup=False)]:
-                a, b = ref_letterbox(im.copy(), **kw), O.letterbox(im.copy(), **kw)
-                assert np.array_equal(a[0], b[0]) and a[1] == b[1] and tuple(a[2]) == tuple(b[2])
+    g = np.load(G / "seam_cases.npz")
+    rng = np.random.default_rng(1)
+    for i, (h, w) in enumerate(g["letterbox/shapes"]):
+        im = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
+        for k, kw in enumerate(ast.literal_eval(str(g["letterbox/kw"]))):
+            b = O.letterbox(im.copy(), **kw)
+            assert b[0].shape == tuple(g[f"letterbox/{i}_{k}/shape"]), (i, k)
+            assert hashlib.sha256(np.ascontiguousarray(b[0]).tobytes()).hexdigest() == str(g[f"letterbox/{i}_{k}/sha256"]), (i, k)
+            assert tuple(b[1]) == tuple(g[f"letterbox/{i}_{k}/ratio"]) and tuple(b[2]) == tuple(g[f"letterbox/{i}_{k}/pad"]), (i, k)

@@ -82,26 +82,23 @@ def test_flat_store_layout_and_groups(name):
 
 
 def test_reference_smart_optimizer_groups_agree():
-    """The same three groups from the REFERENCE's smart_optimizer run on the nn.Module facade (when the reference is around)."""
-    import ref_shim
-
-    if not ref_shim.reference_available():
-        pytest.skip("reference not staged")
-    ref_shim.install()
-    from utils.torch_utils import smart_optimizer
+    """The same three groups as the REFERENCE's smart_optimizer forms (tests/golden/seam_cases.npz: parameter names per
+    group and each group's weight decay), on the nn.Module facade's parameters."""
+    import numpy as np
 
     from yolov3_b200 import params as P
     from yolov3_b200.module import DetectionModel
 
+    g = np.load(ROOT / "tests" / "golden" / "seam_cases.npz")
     dm = DetectionModel(CFG / "yolov3-tiny.yaml", device="cpu")
     st = dm.core.store()
-    opt = smart_optimizer(dm, "SGD", lr=0.01, momentum=0.937, decay=5e-4)
+    named = dict(dm.named_parameters())
     by_ptr = {st.views[n].data_ptr(): n for n in st.order if st.slots[n].group != P.G_FROZEN}
     got = {}
-    for grp, tag in zip(opt.param_groups, (P.G_BIAS, P.G_DECAY, P.G_BN)):  # smart_optimizer: g2 first, then g0 (decay), g1
-        for p in grp["params"]:
-            got[by_ptr[p.data_ptr()]] = tag
-        assert (grp["weight_decay"] > 0) == (tag == P.G_DECAY)
+    for gi, tag in enumerate((P.G_BIAS, P.G_DECAY, P.G_BN)):  # smart_optimizer: g2 first, then g0 (decay), g1
+        for name in g[f"optim/yolov3-tiny/{gi}/names"]:
+            got[by_ptr[named[str(name)].data_ptr()]] = tag
+        assert (g[f"optim/yolov3-tiny/{gi}/hyp"][3] > 0) == (tag == P.G_DECAY)
     assert got == {n: st.slots[n].group for n in by_ptr.values()}
 
 
