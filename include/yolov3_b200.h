@@ -390,6 +390,37 @@ int y3_val_match(const float* det, const int32_t* det_count, int32_t bs, int32_t
                  int32_t* overflow, y3_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
+ * Validation metrics (csrc/y3_metrics.cu).
+ * y3_ap_per_class: ap_per_class + compute_ap (utils/metrics.py:22-120, val.py:424-426).  Row i (0 <= i < n) is
+ *   (conf[i * conf_stride], cls[i * cls_stride], tp[i * niou + 0..niou)); with det_count, row i is valid iff
+ *   i % rows_per_image < det_count[i / rows_per_image] (the padded nms_batched / process_batch_batched layout read in place),
+ *   without it every row is.  Target classes: target_cls[k * target_stride], k < n_targets.  Classes are integral values in
+ *   [0, nc); others are counted in status and ignored.  Outputs are indexed by class id: ap[nc, niou], p, r, f1, tp_out, fp_out
+ *   [nc] (float64, at the F1 index), nt[nc] label counts, present[nc] (the class occurs in the targets: the reference's
+ *   unique_classes; other rows are zero), f1_index[1], status[3] = (valid rows with a bad class, targets with a bad class,
+ *   curves whose true positives exceed their labels: outside the reference's contract, their AP is unspecified).
+ *   Order: class, conf descending, then row — stable, where the reference's argsort is not (bit-equal confidences).
+ *   AP is bit-identical to the reference (np.interp and numpy's pairwise trapezoid restated in double, no contraction);
+ *   p / r / f1 differ at most by the reference's smooth(), which sums through BLAS.  niou <= 64, nc <= 65535.
+ *   workspace: >= y3_ap_per_class_workspace_bytes(n, n_targets, niou, nc) bytes (device). */
+int64_t y3_ap_per_class_workspace_bytes(int64_t n, int64_t n_targets, int32_t niou, int32_t nc);
+int y3_ap_per_class(const float* conf, int64_t conf_stride, const float* cls, int64_t cls_stride, const uint8_t* tp, int32_t niou,
+                    int64_t n, const int32_t* det_count, int64_t rows_per_image, const float* target_cls, int64_t target_stride,
+                    int64_t n_targets, int32_t nc, double eps, void* workspace, int64_t workspace_bytes, double* ap, double* p,
+                    double* r, double* f1, double* tp_out, double* fp_out, int64_t* nt, uint8_t* present, int32_t* f1_index,
+                    int32_t* status, y3_stream_t stream);
+/* y3_confusion_update: ConfusionMatrix.process_batch (utils/metrics.py:134-178) for every image of a padded batch, accumulated
+ *   into matrix[(nc+1) * (nc+1)] (int64, [pred][true], background last; integer atomics).  det [bs, det_stride, 6] (xyxy, conf,
+ *   cls) + det_count[bs] (NULL: max_det each; <= 0: the detections=None call), labels [nl, 6] = (image, cls, xyxy).  Detections
+ *   with conf > conf_thres; pairs with IoU > iou_thres (y3_val_match's IoU, eps 1e-7); each detection keeps its best label, each
+ *   label its best detection among those (bit-equal IoU: lower label, then lower detection index).  Unmatched detections count
+ *   as background only when the image has a match (the reference's quirk).  Class ids are truncated (tensor.int()); ids outside
+ *   [0, nc) are counted in status[0], labels beyond 1024 in one image in status[1] (both accumulate). */
+int y3_confusion_update(const float* det, const int32_t* det_count, int32_t bs, int32_t max_det, int32_t det_stride,
+                        const float* labels, int32_t nl, int32_t nc, float conf_thres, float iou_thres, float eps, int64_t* matrix,
+                        int32_t* status, y3_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
  * Optimizer step over ONE flat fp32 parameter buffer (train.py:411-421: clip_grad_norm_(10.0), SGD-nesterov with the three
  * parameter groups of smart_optimizer utils/torch_utils.py:207-237, ModelEMA.update) — csrc/y3_optim.cu.
  * Layout contract: every parameter occupies a slot whose length is a multiple of 256 elements; group[i] is the group of

@@ -10,6 +10,7 @@ the C ABI in ``include/yolov3_b200.h``; there is no CPU or PyTorch fallback.
     scale_boxes, clip_boxes    utils/general.py:613-626
     box_iou                    utils/metrics.py:10
     process_batch              val.py:147
+    ap_per_class, ConfusionMatrix   utils/metrics.py:22, :124 (ap_per_class_batched: the sync-free padded form)
     ComputeLoss                utils/loss.py:98
     letterbox                  utils/augmentations.py:104 (preprocess.preprocess: + utils/dataloaders.py:308-310 layout step)
     forward_augment, Ensemble, attempt_load   models/yolo.py:239-280, models/experimental.py:74-136
@@ -27,6 +28,7 @@ _EXPORTS = {
     "ComputeLoss": "loss", "process_batch": "val", "process_batch_batched": "val", "letterbox": "preprocess",
     "forward_augment": "tta", "Ensemble": "tta", "attempt_load": "tta", "DDP": "parallel",
     "scale_loss": "parallel", "convert_sync_batchnorm": "parallel", "SGD": "optim", "ModelEMA": "optim", "Pipeline": "pipeline",
+    "ap_per_class": "metrics", "ap_per_class_batched": "metrics", "ConfusionMatrix": "metrics",
 }
 __all__ = sorted(_EXPORTS)
 

@@ -193,6 +193,10 @@ def _declare(lib):
         "y3_scale_img_f32": ([vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, C.c_float, vp, vp], C.c_int),
         "y3_tta_merge": ([vp, i32, i32, i32, i32, i32, C.c_float, i32, C.c_float, vp, i32, i32, vp], C.c_int),
         "y3_val_match": ([vp, vp, i32, i32, i32, vp, i32, vp, i32, C.c_float, vp, vp, vp], C.c_int),
+        "y3_ap_per_class_workspace_bytes": ([C.c_int64, C.c_int64, i32, i32], C.c_int64),
+        "y3_ap_per_class": ([vp, C.c_int64, vp, C.c_int64, vp, i32, C.c_int64, vp, C.c_int64, vp, C.c_int64, C.c_int64, i32,
+                             C.c_double, vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp], C.c_int),
+        "y3_confusion_update": ([vp, vp, i32, i32, i32, vp, i32, i32, C.c_float, C.c_float, C.c_float, vp, vp, vp], C.c_int),
         "y3_sumsq_blocks": ([], i32),
         "y3_grad_sumsq": ([vp, C.c_int64, vp, vp, vp], C.c_int),
         "y3_sgd_step": ([vp, vp, vp, vp, vp, C.c_int64, vp, vp, vp], C.c_int),

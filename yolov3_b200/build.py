@@ -13,7 +13,7 @@ LIB = PKG / "libyolov3_b200.so"
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-diag-suppress", "177",
               "--use_fast_math", "-shared"]
 # kernels whose arithmetic must match the reference bit for bit are compiled without fast-math / FMA contraction
-EXACT_SOURCES = {"y3_nms.cu", "y3_detect.cu", "y3_loss.cu", "y3_iou.cu", "y3_val.cu", "y3_pre.cu", "y3_tta.cu"}
+EXACT_SOURCES = {"y3_nms.cu", "y3_detect.cu", "y3_loss.cu", "y3_iou.cu", "y3_val.cu", "y3_metrics.cu", "y3_pre.cu", "y3_tta.cu"}
 
 
 def nvcc_path() -> str:

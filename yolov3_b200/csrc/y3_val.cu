@@ -11,6 +11,7 @@
 // IoU arithmetic is y3_box_iou's (separately rounded fp32, the reference's operand order), so `>= t` decides identically.
 // Ties (two same-class labels with bit-equal IoU for one detection): the lower label index wins; numpy's argsort is
 // unstable there, like the NMS tie rule (DESIGN.md section 2).
+#include "y3_box.cuh"  // iou_ld (a = label box, b = detection box)
 #include "y3_common.cuh"
 #include "y3_internal.h"
 
@@ -31,15 +32,6 @@ struct ValArgs {
   uint8_t* correct;        // [bs, max_det, niou]
   int* overflow;           // optional [bs]: labels of the image beyond kValMaxLabels (ignored by the matching)
 };
-
-__device__ __forceinline__ float iou_ld(const float4& a, const float4& b, float eps) {  // a = label box, b = detection box
-  const float w = fmaxf(__fsub_rn(fminf(a.z, b.z), fmaxf(a.x, b.x)), 0.0f);
-  const float h = fmaxf(__fsub_rn(fminf(a.w, b.w), fmaxf(a.y, b.y)), 0.0f);
-  const float inter = __fmul_rn(w, h);
-  const float a1 = __fmul_rn(__fsub_rn(a.z, a.x), __fsub_rn(a.w, a.y));
-  const float a2 = __fmul_rn(__fsub_rn(b.z, b.x), __fsub_rn(b.w, b.y));
-  return __fdiv_rn(inter, __fadd_rn(__fsub_rn(__fadd_rn(a1, a2), inter), eps));
-}
 
 __global__ void __launch_bounds__(256) val_match_kernel(const ValArgs p) {
   __shared__ float4 s_box[kValMaxLabels];
