@@ -694,7 +694,9 @@ def build_targets(shapes, targets, anchors, anchor_t=4.0):
         gxy, gwh, a = t[:, 2:4], t[:, 4:6], t[:, 6].long()
         gij = (gxy - offsets).long()
         gi, gj = gij[:, 0].clamp(0, nx - 1), gij[:, 1].clamp(0, ny - 1)
-        # NB reference clamps gj/gi in place AFTER gij is used for tbox (loss.py:239-240): tbox uses unclamped gij
+        # the reference's gi, gj are views of gij and are clamped in place (loss.py:236-239) one statement before tbox is
+        # formed (:240), so tbox uses the CLAMPED indices: a centre at x = 1.0 gives tx = 1.0 in cell nx - 1, not 0.0
+        gij = torch.stack((gi, gj), 1)
         out.append(dict(b=b, a=a, gj=gj, gi=gi, tbox=torch.cat((gxy - gij, gwh), 1), anch=anchors[i][a], tcls=c))
     return out
 

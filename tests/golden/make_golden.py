@@ -2,7 +2,7 @@
 imported unmodified through oracle/ref_shim.py) on seeded inputs, and assert that the CPU oracle (oracle/yolo_oracle.py)
 agrees with it.
 
-    python tests/golden/make_golden.py --reference <checkout> [iou nms loss forward scale val tta seam]
+    python tests/golden/make_golden.py --reference <checkout> [iou nms loss loss_edges forward scale val tta seam]
 
 The fixtures it writes are committed; the tests compare against them and never read the reference.
 
@@ -10,6 +10,7 @@ What is pinned (SURVEY.md Appendix D):
   forward_<model>.npz   Model.forward (fused and unfused) -> z, raw p_i, layer taps      (models/yolo.py:135-147, 89-123)
   nms_cases.npz         non_max_suppression outputs for a sweep + adversarial cases       (utils/general.py:630-750)
   loss_cases.npz        ComputeLoss loss / loss_items / dL/dp and build_targets           (utils/loss.py:131-244)
+  loss_edge_cases.npz   the same on the fp32 boundaries of build_targets, nc 1/2, nl 2/5, na 6, hyps (see gen_loss_edges)
   iou_cases.npz         box_iou, bbox_iou(CIoU) values                                    (ultralytics, via shim)
   val_cases.npz         val.process_batch correct[N,10] on seeded detections / labels     (val.py:147-188)
   tta_cases.npz         Model.forward(x, augment=True) rows (scale / flip views merged)    (models/yolo.py:239-280)
@@ -251,6 +252,225 @@ def gen_loss():
     np.savez_compressed(OUT / "loss_cases.npz", **store)
 
 
+# ---------------------------------------------------------------------------------------------------------------------- loss edges
+# Anchors in pixels per level, as in the model yamls; divided by the stride they are the grid units the loss sees.
+ANCHORS_PX = {
+    "yolov3": (((10, 13), (16, 30), (33, 23)), ((30, 61), (62, 45), (59, 119)), ((116, 90), (156, 198), (373, 326))),
+    "yolov3-tiny": (((10, 14), (23, 27), (37, 58)), ((81, 82), (135, 169), (344, 319))),
+    # the ABI maxima: 5 levels x 6 anchors (P3-P7), growing 1.5x per level so that small images match on every level
+    "p3p7x6": tuple(tuple((round(w * 1.5**l), round(h * 1.5**l)) for w, h in ((10, 13), (16, 30), (33, 23), (30, 61),
+                                                                              (62, 45), (59, 119))) for l in range(5)),
+}
+STRIDES = {"yolov3": (8, 16, 32), "yolov3-tiny": (16, 32), "p3p7x6": (8, 16, 32, 64, 128)}
+
+
+def grid_anchors(kind):
+    return torch.tensor(ANCHORS_PX[kind], dtype=torch.float32) / torch.tensor(STRIDES[kind], dtype=torch.float32)[:, None, None]
+
+
+def f32(v):
+    return np.float32(v)
+
+
+def f32_preimage(fn, want, start, span=256):
+    """The float32 x nearest to `start` with fn(x) == want (fn evaluated in float32), searched over +-span ulps."""
+    x0 = f32(start)
+    up, down = x0, x0
+    for _ in range(span):
+        for x in (up, down):
+            if fn(x) == f32(want):
+                return x
+        up, down = np.nextafter(up, f32(np.inf)), np.nextafter(down, f32(-np.inf))
+    raise AssertionError(f"no float32 preimage of {want} near {start}")
+
+
+def f32_straddle(fn, want, start, span=4096):
+    """Adjacent float32 inputs a < b near `start` with fn(a) < want <= fn(b) or fn(a) >= want > fn(b) (fn in float32)."""
+    x = f32(start)
+    below = fn(x) < f32(want)
+    for to in (f32(np.inf), f32(-np.inf)):
+        v = x
+        for _ in range(span):
+            n = np.nextafter(v, to)
+            if (fn(n) < f32(want)) != below:
+                return (v, n) if to > 0 else (n, v)
+            v = n
+    raise AssertionError(f"fn does not cross {want} near {start}")
+
+
+def f32_neighbours(fn, x):
+    """The float32 inputs nearest to x, below and above, at which fn (evaluated in float32) takes a different value."""
+    out = []
+    for to in (f32(-np.inf), f32(np.inf)):
+        v = x
+        while fn(v) == fn(x):
+            v = np.nextafter(v, to)
+        out.append(v)
+    return tuple(out)
+
+
+def edge_targets(family, kind, imgsz, nc=80, bs=2, anchor_t=4.0):
+    """Target rows [nt, 6] (img, cls, x, y, w, h) that sit on the fp32 boundaries of build_targets (utils/loss.py:207-240)
+    for the grids of `kind` at image size `imgsz` = (h, w).  Boxes are 40 px unless the family needs otherwise: the wh
+    ratio to an anchor does not depend on the level (w * imgsz / anchor_px), and 40 px passes anchor_t = 4 on every level
+    of yolov3, so a centre on the image edge is matched, and clamped, on every level."""
+    H, W = imgsz
+    grids = [(H // s, W // s) for s in STRIDES[kind]]
+    bw, bh = f32(40 / W), f32(40 / H)
+    rows = []
+
+    def row(b, c, x, y, w=bw, h=bh):
+        rows.append([b, c % nc, x, y, w, h])
+
+    if family == "image_edge":
+        for b in range(bs):
+            for k, (x, y) in enumerate([(0.0, 0.0), (1.0, 1.0), (0.0, 1.0), (1.0, 0.0), (0.4, 1.0), (1.0, 0.4),
+                                        (0.0, 0.55), (0.7, 0.0)]):
+                row(b, 3 + k + b, x, y)
+    elif family == "cell_borders":
+        ks = (1, 2, 3, 4, 6, 8, 13, 16, 22, 32, 37, 48, 58, 60, 62, 63)  # x, y = k / 64: gxy % 1 lands on 0, .25, .5, .75
+        for i, kx in enumerate(ks):
+            row(i % bs, i, kx / 64, ks[(i * 7 + 3) % len(ks)] / 64)
+        for ny, nx in grids:  # gxy == 1.0 and gxi == n - gxy == 1.0 exactly, which the strict '> 1' rejects
+            x1 = f32_preimage(lambda v: v * f32(nx), 1.0, 1.0 / nx)
+            y1 = f32_preimage(lambda v: v * f32(ny), 1.0, 1.0 / ny)
+            xn = f32_preimage(lambda v: f32(nx) - v * f32(nx), 1.0, (nx - 1.0) / nx)
+            yn = f32_preimage(lambda v: f32(ny) - v * f32(ny), 1.0, (ny - 1.0) / ny)
+            xh = f32_preimage(lambda v: v * f32(nx), nx // 2 + 0.5, (nx // 2 + 0.5) / nx)  # gxy % 1 == 0.5 exactly
+            for b, (x, y) in enumerate([(x1, y1), (xn, yn), (x1, yn), (xh, 0.5), (0.5, y1)]):
+                row(b % bs, 7 * b + nx, x, y)
+    elif family == "anchor_ratio":
+        t = f32(anchor_t)
+        anchors = grid_anchors(kind).numpy()
+        for l, (ny, nx) in enumerate(grids):
+            a = (l * 2 + 1) % anchors.shape[1]
+            aw, ah = anchors[l, a]
+            h = f32(ah / f32(ny))  # gh / ah == 1: the w side decides
+            r_side = lambda v: (v * f32(nx)) / aw  # noqa: E731
+            inv_side = lambda v: f32(1) / ((v * f32(nx)) / aw)  # noqa: E731
+            for side, (fn, start) in enumerate(((r_side, float(t) * aw / nx), (inv_side, aw / (float(t) * nx)))):
+                # the two fp32 inputs whose ratios straddle anchor_t; where one of them is exactly anchor_t (rejected), also
+                # the nearest ratios either side of it that fp32 can reach
+                ws = list(f32_straddle(fn, t, start))
+                ws += [v for w in ws if fn(w) == t for v in f32_neighbours(fn, w)]
+                for v in ws:
+                    row(l % bs, 10 * l + side, 0.3 + 0.1 * l, 0.6 - 0.2 * side, v, h)
+    elif family == "shared_cells":
+        x, y = 0.3 + 1 / 256, 0.6 + 1 / 256  # inside one cell on every level, away from the cell borders
+        row(0, 5, x, y)
+        row(0, 5, x, y)  # the same target twice
+        row(0, 7, x + 1 / 1024, y, bw * 1.1)  # same cell, different class
+        row(0, 9, x - 1 / 1024, y + 1 / 1024, bw * 0.95, bh * 1.05)  # >= 3 matches on the cell (and on its neighbours)
+        gx0 = grids[0][1]
+        row(1, 11, (3 + 0.25) / gx0, 0.5 + 0.25 / grids[0][0])  # frac .25 -> also matched one cell to the left ...
+        row(1, 12, (2 + 0.6) / gx0, 0.5 + 0.25 / grids[0][0], bw * 1.2)  # ... which is this target's own cell
+    else:
+        raise KeyError(family)
+    return torch.tensor(rows, dtype=torch.float32).reshape(-1, 6)
+
+
+def random_targets(bs, nc, seed, per_image=6, empty=()):
+    """synth_targets-like rows with a given number of targets per image; images in `empty` get none."""
+    g = torch.Generator().manual_seed(seed)
+    t = O.synth_targets(bs, nc=nc, seed=seed)
+    keep = torch.tensor([int(b) not in empty for b in t[:, 0].tolist()], dtype=torch.bool)
+    t = t[keep]
+    return t[torch.randperm(len(t), generator=g)[: per_image * bs]] if per_image else t
+
+
+def loss_edge_case_list():
+    """(name, spec) for loss_edge_cases.npz.  spec: kind (anchor set), imgsz (h, w), bs, nc, hyp overrides, targets builder,
+    logit saturation.  Small images, so that repeated writes to a cell stay few and the reference's tobj is well defined."""
+    return [
+        ("image_edge", dict(kind="yolov3", imgsz=(128, 128), bs=2, nc=80, fam="image_edge")),
+        ("image_edge_rect", dict(kind="yolov3", imgsz=(96, 160), bs=2, nc=80, fam="image_edge")),
+        ("cell_borders", dict(kind="yolov3", imgsz=(128, 128), bs=2, nc=80, fam="cell_borders")),
+        ("cell_borders_640", dict(kind="yolov3", imgsz=(640, 640), bs=1, nc=4, fam="cell_borders")),
+        ("anchor_ratio", dict(kind="yolov3", imgsz=(128, 128), bs=3, nc=80, fam="anchor_ratio")),
+        ("anchor_ratio_t291", dict(kind="yolov3", imgsz=(128, 128), bs=3, nc=80, fam="anchor_ratio", hyp=dict(anchor_t=2.91))),
+        ("shared_cells", dict(kind="yolov3", imgsz=(128, 128), bs=2, nc=80, fam="shared_cells")),
+        ("nc1_smoothing", dict(kind="yolov3", imgsz=(128, 128), bs=2, nc=1, fam="random",
+                               hyp=dict(label_smoothing=0.1, obj_pw=1.3))),
+        ("nc2_hyps", dict(kind="yolov3", imgsz=(128, 128), bs=2, nc=2, fam="random",
+                          hyp=dict(label_smoothing=0.1, cls_pw=1.7, obj_pw=0.6))),
+        ("tiny_nl2", dict(kind="yolov3-tiny", imgsz=(128, 96), bs=2, nc=80, fam="random")),
+        ("abi_max_nl5_na6", dict(kind="p3p7x6", imgsz=(256, 256), bs=1, nc=6, fam="random")),
+        ("rect_empty_images", dict(kind="yolov3", imgsz=(96, 160), bs=3, nc=80, fam="random", empty=(1,))),
+        ("saturated", dict(kind="yolov3", imgsz=(128, 128), bs=2, nc=80, fam="random", sat=12.0)),
+    ]
+
+
+def loss_edge_inputs(spec, seed):
+    """(p list, targets, anchors [nl, na, 2] grid units, hyp) for one edge case."""
+    kind, (H, W), bs, nc = spec["kind"], spec["imgsz"], spec["bs"], spec["nc"]
+    hyp = O.scaled_hyp(nl=len(STRIDES[kind]), nc=nc, imgsz=max(H, W))
+    hyp.update(spec.get("hyp", {}))
+    if spec["fam"] == "random":
+        t = random_targets(bs, nc, seed, per_image=4, empty=spec.get("empty", ()))
+    else:
+        t = edge_targets(spec["fam"], kind, (H, W), nc=nc, bs=bs, anchor_t=hyp["anchor_t"])
+    anchors = grid_anchors(kind)
+    g = torch.Generator().manual_seed(300 + seed)
+    p = [torch.randn(bs, anchors.shape[1], H // s, W // s, nc + 5, generator=g) for s in STRIDES[kind]]
+    if spec.get("sat"):  # logits at +-sat: each entry's sign drawn at random (tw/th pushed to -sat would underflow pwh)
+        for x in p:
+            sgn = torch.where(torch.rand(x.shape, generator=g) < 0.5, -1.0, 1.0)
+            x.copy_(torch.where(torch.rand(x.shape, generator=g) < 0.5, sgn * spec["sat"], x))
+            x[..., 2:4] = x[..., 2:4].abs().clamp(max=3.0)  # pwh = (2 sigmoid)^2 anchor stays away from 0 (0/0 in CIoU)
+    return p, t, anchors, hyp
+
+
+class _RefLossModel(torch.nn.Module):
+    """What the reference's ComputeLoss reads from a model: a parameter (for the device), .hyp and model[-1] = Detect."""
+
+    def __init__(self, anchors, nc, strides, hyp):
+        super().__init__()
+        from types import SimpleNamespace
+
+        self.w = torch.nn.Parameter(torch.zeros(1))
+        self.hyp = hyp
+        self.model = [SimpleNamespace(nl=anchors.shape[0], na=anchors.shape[1], nc=nc, anchors=anchors,
+                                      stride=torch.tensor(strides, dtype=torch.float32))]
+
+
+def gen_loss_edges():
+    """loss_edge_cases.npz: the reference's ComputeLoss on the fp32 boundaries of build_targets, asserted against the oracle."""
+    from utils.loss import ComputeLoss  # reference
+
+    store = {}
+    for ci, (name, spec) in enumerate(loss_edge_case_list()):
+        p, t, anchors, hyp = loss_edge_inputs(spec, ci)
+        nc = spec["nc"]
+        cl = ComputeLoss(_RefLossModel(anchors, nc, STRIDES[spec["kind"]], hyp))
+        pr = [x.clone().requires_grad_(True) for x in p]
+        loss, items = cl(pr, t.clone())
+        loss.backward()
+        po = [x.clone().requires_grad_(True) for x in p]
+        lo, io = O.compute_loss(po, t.clone(), anchors, hyp, nc=nc)
+        lo.backward()
+        assert torch.allclose(loss, lo, rtol=1e-5, atol=1e-6), (name, loss, lo)
+        assert torch.allclose(items, io, rtol=1e-5, atol=1e-6), (name, items, io)
+        for a, b in zip(pr, po):
+            assert torch.allclose(a.grad, b.grad, rtol=1e-4, atol=1e-7), (name, (a.grad - b.grad).abs().max())
+        tcls, tbox, indices, anch = cl.build_targets(pr, t.clone())
+        bt = O.build_targets([tuple(x.shape) for x in p], t, anchors, hyp["anchor_t"])
+        for i in range(len(p)):
+            assert torch.equal(tcls[i], bt[i]["tcls"]) and torch.allclose(tbox[i], bt[i]["tbox"]), (name, i)
+            for a, k in zip(indices[i], ("b", "a", "gj", "gi")):
+                assert torch.equal(a, bt[i][k]), (name, i, k)
+            assert torch.equal(anch[i], bt[i]["anch"])
+            store[f"{name}/bt{i}"] = torch.cat(
+                (torch.stack([x.float() for x in indices[i]], 1), tbox[i], anch[i], tcls[i][:, None].float()), 1).numpy()
+        store[f"{name}/loss"], store[f"{name}/items"] = loss.detach().numpy(), items.numpy()
+        for i, a in enumerate(pr):
+            store[f"{name}/grad{i}"] = a.grad.numpy()
+        store[f"{name}/targets"], store[f"{name}/hyp"] = t.numpy(), np.array(repr(hyp))
+        store[f"{name}/seed"] = np.array(ci)
+        print("loss_edges", name, len(t), "targets", [len(x) for x in tcls], "matches", float(loss), items.tolist())
+    store["cases"] = np.array([n for n, _ in loss_edge_case_list()])
+    np.savez_compressed(OUT / "loss_edge_cases.npz", **store)
+
+
 def gen_iou():
     from utils.metrics import box_iou  # reference re-export (shim restatement of the ultralytics formula)
     import torchvision
@@ -424,7 +644,7 @@ if __name__ == "__main__":
     assert ref_shim.reference_available(), "pass --reference <checkout of ultralytics/yolov3 @ 97b87b1>"
     ref_shim.install()
     torch.set_num_threads(8)
-    which = args or ["iou", "nms", "loss", "forward", "scale", "val", "tta", "seam"]
+    which = args or ["iou", "nms", "loss", "loss_edges", "forward", "scale", "val", "tta", "seam"]
     if "seam" in which:
         gen_seam()
     if "tta" in which:
@@ -439,5 +659,7 @@ if __name__ == "__main__":
         gen_nms()
     if "loss" in which:
         gen_loss()
+    if "loss_edges" in which:
+        gen_loss_edges()
     if "forward" in which:
         gen_forward()

@@ -73,8 +73,8 @@ __global__ void __launch_bounds__(256) loss_match_kernel(const LossArgs p) {
   mt.a = a;
   mt.gi = min(max(gi0, 0), d.nx[l] - 1);
   mt.gj = min(max(gj0, 0), d.ny[l] - 1);
-  mt.tx = gx - static_cast<float>(gi0);
-  mt.ty = gy - static_cast<float>(gj0);
+  mt.tx = gx - static_cast<float>(mt.gi);  // tbox uses the CLAMPED indices: the reference clamps gij in place through
+  mt.ty = gy - static_cast<float>(mt.gj);  // its gi/gj views one statement before it forms gxy - gij (loss.py:236-240)
   mt.tw = gw;
   mt.th = gh;
   mt.aw = aw;

@@ -58,6 +58,9 @@ class ComputeLoss:
         self.balance = {3: [4.0, 1.0, 0.4]}.get(m.nl, [4.0, 1.0, 0.25, 0.06, 0.02])  # utils/loss.py:122
         self.gr, self.autobalance = 1.0, False
         self.na, self.nc, self.nl = m.na, m.nc, m.nl
+        if not (1 <= self.nl <= _lib.MAX_LEVELS and 1 <= self.na <= _lib.MAX_ANCHORS):
+            raise ValueError(f"loss: nl={self.nl}, na={self.na}; the kernel takes 1..{_lib.MAX_LEVELS} levels of "
+                             f"1..{_lib.MAX_ANCHORS} anchors")
         self.anchors = m.anchors.detach().float().cpu()
         self._ws = None
 

@@ -16,7 +16,10 @@ Parameters, gradients and the bf16 weight copy live in ONE flat buffer each (``p
 all weights with two launches, the backward writes every gradient in place, and the data-parallel exchange all-reduces
 contiguous ranges of the gradient buffer on a side stream while the remaining layers are still being back-propagated
 (``parallel.DDP``; reference: DistributedDataParallel buckets, utils/torch_utils.py:60-72).  Every reduction is two-stage
-with a fixed summation order — no floating-point atomics — except the split-K wgrad (``deterministic=True`` removes that too).
+with a fixed summation order — no floating-point atomics — except the split-K wgrad (``deterministic=True`` removes that too)
+and the loss (csrc/y3_loss.cu): it adds the dL/dp of matches that share a cell with float atomics, so on a cell with three
+or more matches the last bits of that gradient depend on the order the adds land in, and it sums its loss terms with
+double atomics before rounding them to float.
 
 ``TrainEngine.forward/backward`` are wrapped in one ``torch.autograd.Function`` so that the reference's
 ``loss.backward(); optimizer.step()`` work unchanged on the fp32 master parameters (``Model.parameters()``).
